@@ -37,6 +37,12 @@ needed between steps.
             config: S bytes per rank, N ranks, same steps/warm-up unless that exceeds ~90 s (then
             capped, and config.steps_capped says so).  The only uses of oracle/ here are that
             baseline, the input generator and the parity checks -- never the measured path.
+
+  --dump-outputs DIR  after the timed steps every rank writes the Allreduce result its last timed step
+            delivered, DIR/allreduce_recv_rank<r>.npy (float32), so that two builds can be compared output
+            for output on the same seeded inputs.  Above DUMP_ELEMS elements over all ranks each rank writes
+            a stratified sample instead: with k = DUMP_ELEMS // N and stride = count // k, element
+            i * stride + o_i for i < k, o_i = np.random.default_rng(SEED).integers(0, stride, k)[i].
 """
 import argparse
 import ctypes
@@ -57,6 +63,7 @@ NVLINK_NOMINAL_GBS = 900.0   # per direction per GPU (B200_PROFILING.md)
 NVLINK_MEASURED_GBS = 770.0  # peer copy measured on this pool (B200_PROFILING.md)
 HBM_FALLBACK_GBS = 6650.0
 BLOCK = 1 << 22              # elements per parity block
+DUMP_ELEMS = 1 << 23         # --dump-outputs: float32 elements over all ranks (32 MiB)
 
 
 def world_from_env(args):
@@ -303,7 +310,12 @@ def main():
     ap.add_argument("--no-nccl", action="store_true")
     ap.add_argument("--deadline", type=int, default=300, help="seconds after which a partial contract line is printed and the run ends")
     ap.add_argument("--nccl-deadline", type=int, default=60, help="seconds the NCCL comparison may take before it is abandoned")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write each rank's Allreduce result of the last timed step to DIR (see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what this library's timed path computed; it does not apply to --impl reference")
     if args.warmup < 3:
         args.warmup = 3
     rank, world, local, addr, addrs = world_from_env(args)
@@ -585,6 +597,20 @@ def main():
     launches = int(lib.b200mpi_launch_count() - l0)
     mpi.Barrier()
     t_step = max_over_ranks(ms.value / 1e3 / args.steps)
+    if args.dump_outputs:  # before anything later in the run writes into recv
+        k = min(count, DUMP_ELEMS // n)
+        idx = np.arange(count, dtype=np.int64)
+        if k < count:
+            stride = count // k
+            idx = np.arange(k, dtype=np.int64) * stride + np.random.default_rng(SEED).integers(0, stride, k)
+        dump = np.empty(idx.size, dtype=dtype)
+        for lo in range(0, count, BLOCK):
+            m = min(BLOCK, count - lo)
+            a, b = np.searchsorted(idx, [lo, lo + m])
+            if b > a:
+                dump[a:b] = recv[lo:lo + m].to_host()[idx[a:b] - lo]
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "allreduce_recv_rank%d.npy" % rank), dump)
 
     algbw = S / t_step / 1e9
     value = algbw * bus

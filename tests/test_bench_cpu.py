@@ -104,6 +104,38 @@ def test_bench_world_of_2_nccl_comparison_block():
     assert c["result_agrees_with_oracle"] is True, c
 
 
+def test_bench_dump_outputs(tmp_path):
+    """--dump-outputs: a world of 1 writes the whole result (a copy of its seeded input), the same on every
+    run; a world of 2 above the size limit writes the documented seeded sample of the sum on each rank."""
+    import numpy as np
+    import bench
+    from oracle import oracle as O
+    count = (1 << 20) // 4
+    for d in ("a", "b"):
+        (rc, out, err), = run_bench(1, "--bytes", str(count * 4), "--steps", "2", "--warmup", "3", "--no-cpu-baseline", "--no-e2e",
+                                    "--dump-outputs", str(tmp_path / d))
+        assert rc == 0, err[-3000:]
+    a, b = np.load(tmp_path / "a" / "allreduce_recv_rank0.npy"), np.load(tmp_path / "b" / "allreduce_recv_rank0.npy")
+    assert a.dtype == np.float32 and np.array_equal(a, O.fill(np.float32, bench.SEED, count)) and np.array_equal(a, b)
+
+    count = bench.DUMP_ELEMS + 3  # two ranks: a sample of every other element, seeded offsets, a tail left out
+    res = run_bench(2, "--bytes", str(count * 4), "--steps", "2", "--warmup", "3", "--no-parity", "--no-e2e", "--no-secondary", "--no-nccl",
+                    "--dump-outputs", str(tmp_path / "c"))
+    assert all(rc == 0 for rc, _, _ in res), "\n".join(e[-2500:] for _, _, e in res)
+    k = bench.DUMP_ELEMS // 2
+    stride = count // k
+    idx = np.arange(k) * stride + np.random.default_rng(bench.SEED).integers(0, stride, k)
+    want = O.allreduce([O.fill(np.float32, bench.SEED + r, count) for r in range(2)])[idx]
+    total = 0
+    for r in range(2):
+        got = np.load(tmp_path / "c" / ("allreduce_recv_rank%d.npy" % r))
+        assert got.dtype == np.float32 and np.array_equal(got, want), r
+        total += got.nbytes
+    assert total <= 64 << 20
+    rc = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, cwd=ROOT).returncode
+    assert rc == 2, "--steps 0 must be refused, not run zero timed steps"
+
+
 def test_bench_deadline_prints_a_partial_line():
     """--deadline in the past: the sections after the timed region are cut short, rank 0 still prints
     the contract keys and every rank exits 0."""
