@@ -16,6 +16,7 @@ sys.path.insert(0, ROOT)
 import mpi_b200 as mpi  # noqa: E402
 from mpi_b200 import _lib as L  # noqa: E402
 from oracle import oracle as O  # noqa: E402
+import _exact as X  # noqa: E402  (tests/, this script's directory)
 
 SEED = 0xB2000000
 DTYPES = {"f32": np.float32, "f64": np.float64, "i64": np.int64}
@@ -850,6 +851,357 @@ def scenario_control_only(a):
         if e.code != L.ERR_NO_DEVICE:
             raise
     return {"checked": 1, "rank": rank, "size": n}
+
+
+# ------------------------------------------------------------------------------------------------
+# Reducing collectives at ragged ownership shapes, every op, checked twice: against tests/_exact.py
+# (order-independent: exact sum + error bound, wrap-around sum, numpy max/min) and bit for bit
+# against the oracle in the order of the kernel that ran.  Every case reports what ran, both
+# verdicts and a SHA-256 of the rank's result; the pytest side compares the digests across ranks.
+# Every rank makes the same calls with the same settings (the grid is part of the call signature).
+SHAPE_ALGOS = (("oneshot", 1, None), ("twoshot_u0", 2, 0), ("twoshot_u1", 2, 1), ("smem", 5, None), ("ring", 3, None))
+OPNAMES = ("sum", "max", "min")
+
+
+def _ok(rc):
+    if rc:
+        raise RuntimeError(L.last_error())
+
+
+def _multicast():
+    info = (L.ctypes.c_size_t(), L.ctypes.c_size_t(), L.ctypes.c_int())
+    L.load().b200mpi_heap_info(L.ctypes.byref(info[0]), L.ctypes.byref(info[1]), L.ctypes.byref(info[2]))
+    return bool(info[2].value)
+
+
+_INPUTS = {}
+
+
+def _inputs(gen, dt, n, count, seed):
+    key = (gen, np.dtype(dt).name, n, count, seed)
+    if key not in _INPUTS:
+        _INPUTS.clear()
+        _INPUTS[key] = X.generate(gen, dt, n, count, seed)
+    return _INPUTS[key]
+
+
+def _row(label, algo, opn, dn, got, xs, want, digest=True):
+    """One reported case: the algorithm that ran, the order-independent verdict, the oracle verdict
+    (None when the order is switch-defined), the result digest."""
+    trace(label)
+    return {"case": label, "algo": L.ALGO_NAMES.get(algo, str(algo)), "op": opn, "dtype": dn,
+            "exact": X.check(got, xs, X.OPS[opn]) if xs is not None else None,
+            "oracle": X.bit_diff(got, want) if want is not None else None,
+            "digest": X.digest(got) if digest else None}
+
+
+def _gen_for(dn, opn, k):
+    if dn == "i64":
+        return "i64"
+    if opn == "sum":
+        return ("signed", "cancel", "uniform01")[k % 3]
+    return ("signed", "cancel")[k % 2]  # max/min over non-negative data would prove little
+
+
+def _allreduce_case(lib, label, dn, opn, gen, count, inplace, kind, seed):
+    rank, n = mpi.Rank(), mpi.Size()
+    dt = DTYPES[dn]
+    op = X.OPS[opn]
+    xs = _inputs(gen, dt, n, count, seed)
+    used = lib.b200mpi_get_algo(L.COLL_ALLREDUCE, count, O.NP2DT[np.dtype(dt)])
+    send = make_buffer(kind, xs[rank])
+    recv = send if inplace else make_buffer(kind, np.zeros(count, dtype=dt))
+    mpi.Allreduce(send, recv, op)
+    got = np.array(read_buffer(recv), copy=True)
+    want, _ = expect_allreduce(xs, op, used, n, count, dt)
+    if not inplace:
+        check_equal(read_buffer(send), xs[rank], label + ": send buffer untouched")
+        free_buffer(recv)
+    free_buffer(send)
+    return _row("%s %s %s %s n=%d count=%d %s%s" % (label, dn, opn, gen, n, count, kind, " inplace" if inplace else ""),
+                used, opn, dn, got, xs, want)
+
+
+def scenario_shapes(a):
+    """Allreduce with every forced P2P algorithm, op and dtype at ragged shapes (own_block_bytes =
+    4 KiB, grids of 1, 3 and all CTAs), at the shuffle / plain one-shot switch, and once at the
+    default 1 MiB block with every rank's share above 1 MiB."""
+    lib = L.load()
+    n = mpi.Size()
+    rows = []
+    _ok(lib.b200mpi_set_param(b"own_block_bytes", X.SMALL_BLOCK))
+    for ai, (aname, aid, unroll) in enumerate(SHAPE_ALGOS):
+        _ok(lib.b200mpi_set_algo(L.COLL_ALLREDUCE, aid))
+        if unroll is not None:
+            _ok(lib.b200mpi_set_param(b"twoshot_unroll", unroll))
+        if aname == "smem" and n not in (2, 4, 8):  # the TMA kernel needs 2, 4 or 8 ranks
+            used = lib.b200mpi_get_algo(L.COLL_ALLREDUCE, X.ragged_counts(n, np.float32)[0], L.F32)
+            if used != L.ALGO_TWOSHOT:
+                raise AssertionError("forced smem at n=%d reports %s, not two-shot" % (n, L.ALGO_NAMES.get(used)))
+            continue
+        for di, dn in enumerate(("f32", "f64", "i64")):
+            counts = X.ragged_counts(n, DTYPES[dn])
+            for oi, opn in enumerate(OPNAMES):
+                gen = _gen_for(dn, opn, ai + di + oi)
+                for inplace in (False, True):
+                    combo = (di * 3 + oi + 3 * inplace) % 6  # every (count, grid) pair 3 times per algorithm
+                    mb = (0, 1, 3)[combo % 3]
+                    _ok(lib.b200mpi_set_max_blocks(mb))
+                    rows.append(_allreduce_case(lib, "shapes %s blocks=%d" % (aname, mb), dn, opn, gen, counts[combo // 3], inplace, "heap",
+                                                SEED + 17 * ai + di))
+        _ok(lib.b200mpi_set_max_blocks(0))
+    # host slices: one case per dtype
+    _ok(lib.b200mpi_set_algo(L.COLL_ALLREDUCE, ALGOS["twoshot"]))
+    for dn in ("f32", "f64", "i64"):
+        rows.append(_allreduce_case(lib, "shapes host twoshot", dn, "sum", _gen_for(dn, "sum", 0), X.ragged_counts(n, DTYPES[dn])[1], False, "host", SEED + 5))
+    _ok(lib.b200mpi_set_param(b"twoshot_unroll", 1))
+    # 4095 / 4096 / 4097 vectors: shuffle one-shot up to 4096, plain one-shot above
+    if n in (4, 8):
+        _ok(lib.b200mpi_set_algo(L.COLL_ALLREDUCE, ALGOS["oneshot"]))
+        for di, dn in enumerate(("f32", "f64", "i64")):
+            for oi, opn in enumerate(OPNAMES):
+                for ci, count in enumerate(X.switch_counts(DTYPES[dn])):
+                    rows.append(_allreduce_case(lib, "switch oneshot", dn, opn, _gen_for(dn, opn, ci + oi), count, (ci + oi) % 2 == 1, "heap", SEED + 9))
+    # the default 1 MiB block: every rank's share above 1 MiB, odd count
+    _ok(lib.b200mpi_set_param(b"own_block_bytes", 1 << 20))
+    for dn, opn in (("f32", "sum"), ("i64", "max")):
+        for ai, (aname, aid, unroll) in enumerate(SHAPE_ALGOS):
+            if aname == "smem" and n not in (2, 4, 8):
+                continue
+            _ok(lib.b200mpi_set_algo(L.COLL_ALLREDUCE, aid))
+            if unroll is not None:
+                _ok(lib.b200mpi_set_param(b"twoshot_unroll", unroll))
+            rows.append(_allreduce_case(lib, "big %s" % aname, dn, opn, _gen_for(dn, opn, 0), X.big_count(n, DTYPES[dn]), ai % 2 == 1, "heap", SEED + 3))
+    _ok(lib.b200mpi_set_param(b"twoshot_unroll", 1))
+    _ok(lib.b200mpi_set_algo(L.COLL_ALLREDUCE, 0))
+    mpi.Barrier()
+    return {"rows": rows}
+
+
+def scenario_reduce_ops(a):
+    """Reduce (every op, roots 0, 1, n-1; in place on the root; NULL recv on non-roots through the
+    C ABI), ReduceScatter (every op, ragged blocks, grids of 1 and all CTAs) and, up to 4 ranks,
+    Allgather in place (send = the caller's block of recv), push and ring, heap and host."""
+    lib = L.load()
+    rank, n = mpi.Rank(), mpi.Size()
+    switch = _multicast()  # Reduce / ReduceScatter sums then go through the switch: no fixed order
+    rows = []
+    _ok(lib.b200mpi_set_param(b"own_block_bytes", X.SMALL_BLOCK))
+    for di, dn in enumerate(("f32", "f64", "i64")):
+        dt = DTYPES[dn]
+        code = O.NP2DT[np.dtype(dt)]
+        count = X.ragged_counts(n, dt)[0]
+        for oi, opn in enumerate(OPNAMES):
+            op = X.OPS[opn]
+            gen = _gen_for(dn, opn, di + oi)
+            xs = _inputs(gen, dt, n, count, SEED + 40 + di)
+            for ri, root in enumerate(sorted({0, 1, n - 1})):
+                mode = ("out", "null", "inplace")[(di + oi + ri) % 3]
+                mb = (0, 1, 3)[(di + 2 * oi + ri) % 3]
+                _ok(lib.b200mpi_set_max_blocks(mb))
+                send = mpi.Alloc(count, dt).copy_from_host(xs[rank])
+                sentinel = np.full(count, -7, dtype=dt)
+                if rank == root:
+                    recv = send if mode == "inplace" else mpi.Alloc(count, dt).copy_from_host(sentinel)
+                else:
+                    recv = None if mode == "null" else mpi.Alloc(count, dt).copy_from_host(sentinel)
+                _ok(lib.b200mpi_reduce(send.ptr, recv.ptr if recv is not None else None, count, code, op, root, L.DEVICE))
+                label = "reduce %s %s %s root=%d %s blocks=%d n=%d count=%d" % (dn, opn, gen, root, mode, mb, n, count)
+                if rank == root:
+                    got = recv.to_host()
+                    exact_order = not (switch and op == X.SUM and dn != "i64" and n >= 4)
+                    want = O.allreduce(xs, op=op, order=O.ORDER_RANK) if exact_order else None
+                    rows.append(_row(label, L.ALGO_TWOSHOT, opn, dn, got, xs, want, digest=False))
+                else:  # the same case on every rank; here the check is that nothing was written
+                    check_equal(send.to_host(), xs[rank], label + ": non-root send untouched")
+                    if recv is not None:
+                        check_equal(recv.to_host(), sentinel, label + ": non-root recv untouched")
+                    rows.append({"case": label, "algo": L.ALGO_NAMES[L.ALGO_TWOSHOT], "op": opn, "dtype": dn, "exact": None, "oracle": None, "digest": None})
+                if recv is not None and recv is not send:
+                    recv.free()
+                send.free()
+        # ReduceScatter: rank j receives block j (of `count`, ragged) reduced over the ranks
+        for ci, count in enumerate(X.ragged_counts(n, dt)):
+            for oi, opn in enumerate(OPNAMES):
+                op = X.OPS[opn]
+                gen = _gen_for(dn, opn, ci + oi)
+                xs = _inputs(gen, dt, n, count * n, SEED + 50 + di)
+                mb = (0, 1)[(ci + oi) % 2]
+                inplace = (di + ci + oi) % 2 == 1
+                _ok(lib.b200mpi_set_max_blocks(mb))
+                send = mpi.Alloc(count * n, dt).copy_from_host(xs[rank])
+                recv = send[rank * count:(rank + 1) * count] if inplace else mpi.Alloc(count, dt)
+                mpi.ReduceScatter(send, recv, op)
+                got = recv.to_host()
+                blocks = [x[rank * count:(rank + 1) * count] for x in xs]
+                exact_order = not (switch and op == X.SUM and dn != "i64")
+                want = O.reduce_scatter(xs, rank, op=op, order=O.ORDER_RANK) if exact_order else None
+                label = "reduce_scatter %s %s %s blocks=%d%s n=%d count=%d" % (dn, opn, gen, mb, " inplace" if inplace else "", n, count)
+                rows.append(_row(label, L.ALGO_TWOSHOT, opn, dn, got, blocks, want, digest=False))
+                if not inplace:
+                    check_equal(send.to_host(), xs[rank], label + ": send untouched")
+                    recv.free()
+                send.free()
+    _ok(lib.b200mpi_set_max_blocks(0))
+    # Allgather in place: the caller's block of recv is the send buffer
+    if n <= 4:
+        for dn in ("f32", "i64"):
+            dt = DTYPES[dn]
+            count = X.ragged_counts(n, dt)[0]
+            xs = _inputs(_gen_for(dn, "sum", 0), dt, n, count, SEED + 60)
+            full = np.concatenate(xs)
+            for ai, algo in enumerate(("oneshot", "ring")):
+                _ok(lib.b200mpi_set_algo(L.COLL_ALLGATHER, ALGOS[algo]))
+                for ki, kind in enumerate(("heap", "host")):
+                    mb = (0, 1)[(ai + ki) % 2]
+                    _ok(lib.b200mpi_set_max_blocks(mb))
+                    init = np.full(count * n, -1, dtype=dt)
+                    init[rank * count:(rank + 1) * count] = xs[rank]
+                    recv = make_buffer(kind, init)
+                    mpi.Allgather(recv[rank * count:(rank + 1) * count], recv)
+                    got = np.array(read_buffer(recv), copy=True)
+                    label = "allgather inplace %s %s %s blocks=%d n=%d count=%d" % (algo, kind, dn, mb, n, count)
+                    row = _row(label, ALGOS[algo], "sum", dn, got, None, full)
+                    row["op"] = "copy"
+                    rows.append(row)
+                    free_buffer(recv)
+        _ok(lib.b200mpi_set_max_blocks(0))
+        _ok(lib.b200mpi_set_algo(L.COLL_ALLGATHER, 0))
+    _ok(lib.b200mpi_set_param(b"own_block_bytes", 1 << 20))
+    mpi.Barrier()
+    return {"rows": rows, "multicast": switch}
+
+
+EDGE_F32 = np.array([np.nan, 0.0, -0.0, np.inf, -np.inf, np.finfo(np.float32).max, -np.finfo(np.float32).max,
+                     2.0 ** -149, -2.0 ** -149, 2.0 ** -130, 1.0, -1.0], dtype=np.float32)
+EDGE_F64 = np.array([np.nan, 0.0, -0.0, np.inf, -np.inf, np.finfo(np.float64).max, -np.finfo(np.float64).max,
+                     2.0 ** -1074, -2.0 ** -1074, 2.0 ** -1050, 1.0, -1.0], dtype=np.float64)
+EDGE_I64 = np.array([-2 ** 63, 2 ** 63 - 1, -2 ** 63 + 1, 2 ** 63 - 2, -1, 0, 1, 42], dtype=np.int64)
+
+
+def edge_inputs(dt, n, count, seed):
+    """Per element, each rank picks a value of the edge set; for floats, the first two elements of
+    ring chunk 1 are set so that the order shows: {x0 = 1, x1 = NaN, rest 1} and {x0 = +0, x1 = -0,
+    rest +0}.  max/min keep the left operand on NaN and ties, so rank order yields 1 and +0 there
+    while the ring, which starts chunk 1 at rank 1, yields NaN and -0."""
+    edge = {np.dtype(np.float32): EDGE_F32, np.dtype(np.float64): EDGE_F64, np.dtype(np.int64): EDGE_I64}[np.dtype(dt)]
+    xs = [edge[(X.splitmix64(seed + r, count) % np.uint64(edge.size)).astype(np.int64)] for r in range(n)]
+    planted = []
+    if np.dtype(dt).kind == "f":
+        e = X.epv(dt)
+        per = -(-(count // e) // n)
+        lo = per * e  # first element of ring chunk 1
+        for k, (first, second, rest) in enumerate(((1.0, np.nan, 1.0), (0.0, -0.0, 0.0))):
+            for r in range(n):
+                xs[r][lo + k] = first if r == 0 else second if r == 1 else rest
+            planted.append(lo + k)
+    return xs, planted
+
+
+def scenario_edge_ops(a):
+    """MAX and MIN over NaN, +-0, +-inf, +-max, subnormals and the int64 extremes, every forced P2P
+    algorithm, bit for bit against the oracle in that algorithm's order."""
+    lib = L.load()
+    rank, n = mpi.Rank(), mpi.Size()
+    rows, pinned = [], 0
+    for ai, (aname, aid, unroll) in enumerate(SHAPE_ALGOS):
+        if aname == "smem" and n not in (2, 4, 8):
+            continue
+        _ok(lib.b200mpi_set_algo(L.COLL_ALLREDUCE, aid))
+        if unroll is not None:
+            _ok(lib.b200mpi_set_param(b"twoshot_unroll", unroll))
+        for dn in ("f32", "f64", "i64"):
+            dt = DTYPES[dn]
+            count = 64 * n * X.epv(dt) + X.epv(dt) - 1  # ring chunks of 64 vectors, a scalar tail
+            xs, planted = edge_inputs(dt, n, count, SEED + 70 + ai)
+            for opn in ("max", "min"):
+                op = X.OPS[opn]
+                used = lib.b200mpi_get_algo(L.COLL_ALLREDUCE, count, O.NP2DT[np.dtype(dt)])
+                send = mpi.Alloc(count, dt).copy_from_host(xs[rank])
+                recv = mpi.Alloc(count, dt)
+                mpi.Allreduce(send, recv, op)
+                got = recv.to_host()
+                send.free()
+                recv.free()
+                want, order = expect_allreduce(xs, op, used, n, count, dt)
+                rows.append(_row("edge %s %s %s n=%d count=%d" % (aname, dn, opn, n, count), used, opn, dn, got, None, want))
+                if used == L.ALGO_RING and planted:
+                    rank_order = O.allreduce(xs, op=op, order=O.ORDER_RANK)
+                    if not X.bit_diff(got[planted], rank_order[planted]):
+                        raise AssertionError("ring %s %s: the planted NaN / -0 elements do not show the ring order" % (dn, opn))
+                    pinned += 1
+    _ok(lib.b200mpi_set_param(b"twoshot_unroll", 1))
+    _ok(lib.b200mpi_set_algo(L.COLL_ALLREDUCE, 0))
+    mpi.Barrier()
+    return {"rows": rows, "ring_order_pinned": pinned}
+
+
+def scenario_oneshot_budget(a):
+    """One CTA per rank: the largest count whose one-shot plan fits in the mid-barrier budget runs
+    one-shot, one vector more runs two-shot; both out of place, then the limit once in place."""
+    import time
+    lib = L.load()
+    rank, n = mpi.Rank(), mpi.Size()
+    _ok(lib.b200mpi_set_max_blocks(1))
+    _ok(lib.b200mpi_set_algo(L.COLL_ALLREDUCE, ALGOS["oneshot"]))
+    lim = X.oneshot_limit(np.float32, n, 1)
+    rows, times = [], {}
+    for count, inplace, expect in ((lim, False, L.ALGO_ONESHOT), (lim + 4, False, L.ALGO_TWOSHOT), (lim, True, L.ALGO_ONESHOT)):
+        used = lib.b200mpi_get_algo(L.COLL_ALLREDUCE, count, L.F32)
+        if used != expect:
+            raise AssertionError("count %d: get_algo reports %s, want %s" % (count, L.ALGO_NAMES.get(used), L.ALGO_NAMES[expect]))
+        mpi.Barrier()
+        t0 = time.time()
+        rows.append(_allreduce_case(lib, "budget", "f32", "sum", "signed", count, inplace, "heap", SEED + 80))
+        times["%d%s" % (count, " inplace" if inplace else "")] = time.time() - t0
+    _ok(lib.b200mpi_set_max_blocks(0))
+    _ok(lib.b200mpi_set_algo(L.COLL_ALLREDUCE, 0))
+    mpi.Barrier()
+    return {"rows": rows, "limit": lim, "seconds": times}
+
+
+def scenario_switch_bound(a):
+    """NVLS and hybrid Allreduce and NVLS ReduceScatter (f32, f64 sums) held to the any-order error
+    bound of tests/_exact.py.  Needs a multicast mapping (one GPU per rank)."""
+    lib = L.load()
+    rank, n = mpi.Rank(), mpi.Size()
+    if not _multicast():
+        raise AssertionError("no multicast mapping: the switch paths cannot run in this world")
+    _ok(lib.b200mpi_set_param(b"hybrid_p2p_permille", 250))
+    _ok(lib.b200mpi_set_param(b"hybrid_min_bytes", 0))
+    rows = []
+    for dn in ("f32", "f64"):
+        dt = DTYPES[dn]
+        for ci, count in enumerate((X.ragged_counts(n, dt)[0], X.big_count(n, dt))):
+            for algo in ("nvls", "hybrid"):
+                _ok(lib.b200mpi_set_algo(L.COLL_ALLREDUCE, ALGOS[algo]))
+                for gi, gen in enumerate(("signed", "cancel", "uniform01")):
+                    xs = _inputs(gen, dt, n, count, SEED + 90 + ci)
+                    used = lib.b200mpi_get_algo(L.COLL_ALLREDUCE, count, O.NP2DT[np.dtype(dt)])
+                    send = mpi.Alloc(count, dt).copy_from_host(xs[rank])
+                    recv = send if gi == 1 else mpi.Alloc(count, dt)  # the cancelling data in place
+                    mpi.Allreduce(send, recv, mpi.SUM)
+                    got = recv.to_host()
+                    if recv is not send:
+                        recv.free()
+                    send.free()
+                    rows.append(_row("switch allreduce %s %s %s n=%d count=%d" % (algo, dn, gen, n, count), used, "sum", dn, got, xs, None))
+            _ok(lib.b200mpi_set_algo(L.COLL_REDUCE_SCATTER, ALGOS["nvls"]))
+            rc = count - count % X.epv(dt)  # whole vectors per block: the switch form
+            for gen in ("signed", "cancel"):
+                xs = _inputs(gen, dt, n, rc * n, SEED + 95 + ci)
+                send = mpi.Alloc(rc * n, dt).copy_from_host(xs[rank])
+                recv = mpi.Alloc(rc, dt)
+                mpi.ReduceScatter(send, recv, mpi.SUM)
+                got = recv.to_host()
+                send.free()
+                recv.free()
+                rows.append(_row("switch reduce_scatter nvls %s %s n=%d count=%d" % (dn, gen, n, rc), L.ALGO_NVLS, "sum", dn, got,
+                                 [x[rank * rc:(rank + 1) * rc] for x in xs], None, digest=False))
+    _ok(lib.b200mpi_set_algo(L.COLL_ALLREDUCE, 0))
+    _ok(lib.b200mpi_set_algo(L.COLL_REDUCE_SCATTER, 0))
+    mpi.Barrier()
+    return {"rows": rows}
 
 
 SCENARIOS = {k[len("scenario_"):]: v for k, v in list(globals().items()) if k.startswith("scenario_")}
